@@ -9,7 +9,10 @@ reference laser_slam/src/laser_track.cpp:466-519) of the next scan of a syntheti
           from pinned host memory (ls_map_push_scan) and reads the 4x4 result + stats back.
   --impl reference : the reference's CPU algorithm (oracle port: kd-tree 1-NN, nth_element trim,
           point-to-plane) on the host cores -- the reference's own libraries are absent (SURVEY.md §8c).
-Prints ONE JSON line on rank 0.
+  --dump-outputs DIR : after the timed steps, write what the resident arm's last timed step returned to its
+          caller, one DIR/<name>.npy per array (see dump_outputs); the inputs depend only on the arguments, so two
+          builds run with the same arguments can be compared output for output.
+Prints ONE JSON line on rank 0.  Writes nothing into the source tree.
 """
 import argparse
 import json
@@ -23,6 +26,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree may be read-only; no __pycache__ next to the sources
 
 # BASELINE.json configs[1] (default) and configs[4] (--config 5): scan size, scans per map, ICP iterations, sensor
 WORKLOADS = {
@@ -238,6 +242,20 @@ def cpu_baseline_sample():
                       f"single-thread (libpointmatcher default): {out[1]:.3f} registrations/s"}
 
 
+# IcpStats fields that say how a registration ended.  The timings (device_ms, build_ms, icp_ms) and the spatial-hash
+# diagnostics (grid_*) describe how it was computed, not what, so two correct builds may differ in them.
+DUMP_STATS = ("iterations", "converged", "max_iter_reached", "last_kept", "last_limit", "used_ratio")
+
+
+def dump_outputs(out_dir, touts, stats):
+    """One registration per track, tracks in order: transforms.npy (B,4,4) float32, the row-major T_ref<-reading each
+    registration returned, and one <field>.npy (B,) float64 per DUMP_STATS field of its IcpStats."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "transforms.npy"), np.ascontiguousarray(touts.reshape(-1, 4, 4).transpose(0, 2, 1)))
+    for f in DUMP_STATS:
+        np.save(os.path.join(out_dir, f"{f}.npy"), np.array([getattr(st, f) for st in stats], np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -253,7 +271,11 @@ def main():
     ap.add_argument("--config", type=int, default=2, choices=(2, 3, 4, 5),
                     help="BASELINE.json workload: 2 scan-to-map ICP (default, the headline metric), 3 batched trajectories "
                          "feeding the shared estimator, 4 pose-graph solve, 5 dense-sensor stress")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the transforms and ICP stats of the last timed step as DIR/<name>.npy (configs 2 and 5)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.config in (3, 4) or args.impl == "reference"):
+        ap.error("--dump-outputs records the GPU scan-to-map registrations: --config 2 or 5, --impl ours")
     if args.config == 4:
         import bench_posegraph
         return bench_posegraph.main(args)
@@ -350,12 +372,14 @@ def main():
             prepared[g].append(mps[g].prepare_begin_batch(probs, prm))
     dev_ms, icp_ms = [], []
     last_touts = [None] * G
+    last_stats = [None] * G
 
     def finish(g, s, record):
         rc, statuses, touts, stats = prepared[g][s][1]()
         if rc != 0 or statuses.any():
             raise RuntimeError(f"registration failed rc={rc} {list(statuses)}")
         last_touts[g] = touts.copy()
+        last_stats[g] = stats   # every prepared step owns its stats array: a reference is enough
         if world > 1 and g == 0:
             share_pose_delta(ls.from_colmajor(touts[0]))
         if record:
@@ -498,7 +522,7 @@ def main():
                     [nrms[t][idxs[t]].data_ptr() for t in range(B)], [N_SCAN] * B), [pose7(tracks[t][1][idxs[t]]) for t in range(B)]
 
         # the same scans as the C-ABI arm's timed steps: its step s registers scan walk(s + K_MAP + 1)
-        n_host = max(3, min(args.steps, 60))
+        n_host = args.steps
         w_host = args.warmup + K_MAP + 1
         hargs = [host_args(s) for s in range(w_host + n_host + 1)]   # marshalled before the clock, like the C-ABI arm's
 
@@ -610,6 +634,8 @@ def main():
     }
     if cpu:
         out["cpu_baseline"] = cpu
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, np.concatenate(last_touts), [st for g in range(G) for st in last_stats[g]])
     print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()

@@ -81,12 +81,9 @@ def test_yaml_chain_reader(ls):
 
 
 def test_reference_default_yaml_is_accepted(ls):
-    """The reference's own chain file must parse (laser_slam/configurations/icp_default.yaml); only read when
-    the reference tree is mounted (never on the GPU box)."""
-    path = "/root/reference/laser_slam/configurations/icp_default.yaml"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not mounted")
-    p = ls.params_from_yaml(open(path).read())
+    """The reference's own chain file must parse: tests/golden/icp_default.yaml is a byte-for-byte copy of
+    laser_slam/configurations/icp_default.yaml from ethz-asl/laser_slam (BSD-3-Clause)."""
+    p = ls.params_from_yaml(open(os.path.join(ROOT, "tests", "golden", "icp_default.yaml")).read())
     assert p.max_iterations == 40 and p.use_differential == 1 and abs(p.trim_ratio - 0.75) < 1e-7
 
 
