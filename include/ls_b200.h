@@ -83,7 +83,8 @@ const char* ls_b200_last_error(const ls_ctx* ctx); /* text of the last failure o
 int ls_b200_version(void);
 /* Cap the number of CTAs the persistent ICP kernel of this context may occupy (0 = all that can be co-resident, the
  * default).  Two contexts that each take half of the device run their cooperative launches side by side, so the map build
- * and host-side staging of one overlap the ICP iterations of the other (bench.py drives two such contexts). */
+ * and host-side staging of one overlap the ICP iterations of the other (bench.py drives two such contexts).  A batch of
+ * more problems than the budget still gets one CTA per problem, so its launch then occupies more CTAs than the budget. */
 int ls_b200_set_icp_cta_budget(ls_ctx* ctx, int ctas);
 int ls_b200_icp_cta_budget(const ls_ctx* ctx); /* CTAs the next launch will use at most */
 /* Number of this library's kernel launches issued on the context so far (bench "gpu_launches"). */
